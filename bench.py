@@ -3,6 +3,7 @@
 configs as secondary legs of the same JSON line.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
+  python bench.py ... --dump-outputs DIR                        # + the last timed step's MSM point as DIR/*.npy
   python bench.py --impl reference [...]                        # CPU arm (oracle port, all host cores)
   torchrun --nproc-per-node N bench.py --gpus N ...             # one rank per GPU
 
@@ -32,6 +33,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the benchmark leaves the tree it runs from untouched (no __pycache__)
 
 import numpy as np  # noqa: E402
 
@@ -374,6 +376,13 @@ def msm_leg(ctx):
     ms, _ = timed_region(ctx, lambda: run_steps(K))
     got = jac_to_affine(C, d_tot[K - 1].cpu().numpy().view(np.uint64))
     assert got == expected_total, "sum over ranks does not match the known-discrete-log oracle"
+    if args.dump_outputs and rank == 0:
+        # the last timed step's point in affine form, which is unique (Jacobian X, Y, Z are not): gnark-crypto's
+        # uncompressed encoding, rows X and Y of 32 big-endian bytes, one exact float64 per byte
+        from oracle import encoding
+        raw = np.frombuffer(encoding.encode_g1(C, got, compressed=False), dtype=np.uint8)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "msm_point_affine.npy"), raw.reshape(2, 32).astype(np.float64))
 
     # ---- end to end through the C ABI with HOST buffers (e2e) -------------------------------------------
     # K x b200_msm_submit_dev (pinned host scalars: H2D on the copy stream, overlapped with the previous MSM), one
@@ -734,7 +743,11 @@ def main():
     ap.add_argument("--bw6-log", type=int, default=24)
     ap.add_argument("--imad-per-add", type=int, default=1360,
                     help="IMAD.WIDE per XYZZ mixed addition of the shipped kernel (static SASS count, profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="CUDA arm: after the timed steps, write the MSM result of the last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     dog = arm_watchdog(WHOLE_RUN_LIMIT_S, code=1)
     if args.impl == "reference":
         run_reference(args)
