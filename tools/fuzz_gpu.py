@@ -7,6 +7,11 @@ cases live in tests/test_gpu_*.py, this tool widens them with sizes and patterns
     python tools/fuzz_gpu.py --seconds 300 --seed 1 > gpurun_out/fuzz_gpu.jsonl
 
 One JSON line per case class at the end (cases run, failures with their reproducer seeds); exit code 1 on any mismatch.
+
+    python tools/fuzz_gpu.py --field 600 --seed 1 > field_soak.jsonl
+
+runs only the field-arithmetic soak instead (every device field template against an independent reference on
+carry-hunting operands, tests/cuda/field_soak.cu; `make` builds tests/_build/libgb200_fieldsoak.so).
 """
 import argparse
 import json
@@ -181,6 +186,70 @@ def case_known_dlog_big(rs, seed):
 BIG_GROUP = 0     # --big-group: 1 / 2 pins the group of the big cases (2: the Fp2 arithmetic)
 
 
+def card_info():
+    """name, power limit and max SM clock of the card the soak runs on (read-only nvidia-smi query)"""
+    import subprocess
+    dev = os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0] or "0"
+    try:
+        out = subprocess.run(["nvidia-smi", "-i", dev, "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=60).stdout.strip().splitlines()
+        name, power, clock = (x.strip() for x in out[0].split(","))
+        return {"gpu": name, "power_limit": power, "max_sm_clock": clock}
+    except Exception as e:              # the numbers stay usable, the card just goes unnamed
+        return {"gpu": "unknown (%r)" % e}
+
+
+def field_soak(seconds, seed, lib_name="libgb200_fieldsoak.so", target=0.25):
+    """--field: tests/cuda/field_soak.cu's fs_soak round-robin over every (field, op, generator) of the device field
+    templates with fresh seeds, product against the independent reference in the same kernel.  Each call is sized from
+    the rate of the previous one to take about `target` seconds.  Prints one header line (card, power limit), one line
+    per (field, op, generator) with samples, mismatches and rate, and the recorded mismatches checked with big ints."""
+    import fieldsoak as fs
+    slib = fs.load(lib_name)
+    head = {"kind": "field_soak", "seed": seed, "seconds": seconds, "lib": lib_name, **card_info()}
+    print(json.dumps(head), flush=True)
+    cases = [(f, op, gen) for f in fs.DEVICE_FIELDS for op in f.ops if op != "reduce_mutant" for gen in fs.gens_for(op)]
+    count = {c: (1 << 12 if c[1] == "inverse" else 1 << 20) for c in cases}
+    tot = {c: {"samples": 0, "mismatches": 0, "seconds": 0.0, "calls": 0} for c in cases}
+    failures = []
+    t0 = last = time.time()
+    rnd = 0
+    while time.time() - t0 < seconds:
+        for c in cases:
+            if time.time() - last >= 30:        # progress line: a long soak keeps writing
+                last = time.time()
+                print(json.dumps({"kind": "field_soak_progress", "elapsed": round(last - t0, 1), "round": rnd,
+                                  "samples": sum(st["samples"] for st in tot.values()),
+                                  "mismatches": sum(st["mismatches"] for st in tot.values())}), flush=True)
+            if time.time() - t0 >= seconds:
+                break
+            f, op, gen = c
+            s = (seed * 1_000_003 + rnd) * 4099 + f.fid
+            t = time.perf_counter()
+            m, recs = fs.soak(slib, f, op, gen, s, count[c])
+            dt = time.perf_counter() - t
+            st = tot[c]
+            st["samples"] += count[c]
+            st["mismatches"] += m
+            st["seconds"] += dt
+            st["calls"] += 1
+            if m:
+                msg = fs.triage(f, op, gen, s, recs, "device")
+                failures.append({"field": f.name, "op": op, "gen": gen, "seed": s, "mismatches": m, "triage": msg})
+                sys.stderr.write(msg + "\n")
+            count[c] = int(min(max(count[c] * target / max(dt, 1e-3), 1 << 10), 1 << 34))
+        rnd += 1
+    for (f, op, gen), st in tot.items():
+        if st["calls"]:
+            print(json.dumps({"kind": "field_soak_case", "field": f.name, "op": op, "gen": gen, **st,
+                              "rate_per_s": st["samples"] / st["seconds"] if st["seconds"] else None}))
+    summ = {"kind": "field_soak_total", "rounds": rnd, "wall_seconds": time.time() - t0,
+            "samples": sum(st["samples"] for st in tot.values()),
+            "mismatches": sum(st["mismatches"] for st in tot.values()), "failures": failures}
+    print(json.dumps(summ))
+    return 1 if summ["mismatches"] else 0
+
+
 CASES = {"msm": (case_msm, 5), "known_dlog_big": (case_known_dlog_big, 0), "ntt": (case_ntt, 3), "compute_h": (case_compute_h, 1), "fixed_base": (case_fixed_base, 1),
          "gather": (case_gather, 1)}
 
@@ -192,7 +261,13 @@ def main():
     ap.add_argument("--only", default="")
     ap.add_argument("--big", type=float, default=0.0, help="weight of the 2^17..2^20 known-discrete-log MSM cases (0 = off)")
     ap.add_argument("--big-group", type=int, default=0, help="pin the group (1 or 2) of the big cases")
+    ap.add_argument("--field", type=float, default=0.0,
+                    help="run only the device field-arithmetic soak for this many seconds (tests/cuda/field_soak.cu)")
+    ap.add_argument("--field-lib", default="libgb200_fieldsoak.so",
+                    help="soak library under tests/_build (libgb200_hostemu.so rehearses --field on a CPU)")
     args = ap.parse_args()
+    if args.field > 0:
+        sys.exit(field_soak(args.field, args.seed, args.field_lib))
     global BIG_GROUP
     BIG_GROUP = args.big_group
     lib.load()
